@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — headline benchmark of the two hot paths (BASELINE.json `metric`).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One "step" is one pass of the hot path over one batch of synthetic input:
   * BLS  (headline, BASELINE configs[2]): bls::verify_signature_sets over 100 000 aggregate attestations x 128 pubkeys per
@@ -19,6 +19,11 @@ per launch (counted by ncu, profiles/r2_counters.json) / its live CUDA-event tim
 peak; the HBM numbers the contract asks for sit under `roofline.hbm` / `roofline.traffic`.
 `--impl reference` times the CPU oracle (oracle/, kind "port": the reference's Rust/blst path cannot be built here) on
 the host cores on a bounded sample OF THE SAME WORKLOAD (same generator, same seed).
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of each hot path returned to its caller
+(rank 0), so that two builds can be compared output for output on the same seeded inputs:
+  bls_verdict.npy     float64 [1]       verdict of the last BLS step (1.0 = every set verified)
+  bls_set_status.npy  float32 [N_SETS]  per-set status of that step (0 = the set entered the batch check, else why it was rejected)
+  state_root.npy      float64 [32]      bytes of the BeaconState root the last tree-hash step produced
 """
 import argparse
 import ctypes as C
@@ -271,6 +276,12 @@ def run_ours(args):
     clocks = sampler.stop()
     assert ok and int(verdict.item()) == 1
     bls_value = N_SETS * world / (bls_ms / 1e3)
+    outputs = {}
+    if args.dump_outputs:
+        # reads back the device verdict and statuses of the last enqueue; the batch is reused below
+        ok_last, status = batch.result(sp, want_status=True)
+        outputs["bls_verdict"] = np.array([float(ok_last)], dtype=np.float64)
+        outputs["bls_set_status"] = status.astype(np.float32)
 
     # e2e: THE PLUGIN CALL lhb200_verify_signature_sets with host buffers (H2D of every input and D2H of the verdict inside)
     offs_np = ab.offsets.copy()
@@ -388,6 +399,7 @@ def run_ours(args):
             if world > 1:   # one all-gather of the 32-byte roots THIS step produced (device pointer, no host hop)
                 mine = torch.as_tensor(DevPtr(d_root, 32), device=dev)
                 dist.all_gather_into_tensor(roots_all, mine)
+        return d_root
 
     for _ in range(W):
         state_step()
@@ -396,10 +408,12 @@ def run_ours(args):
     with torch.cuda.stream(stream):
         e0.record(stream)
     for _ in range(K):
-        state_step()
+        d_root = state_step()
     with torch.cuda.stream(stream):
         e1.record(stream)
     barrier()
+    if args.dump_outputs:
+        outputs["state_root"] = torch.as_tensor(DevPtr(d_root, 32), device=dev).cpu().numpy().astype(np.float64)
     st_dom = st.dominant_kernel_ms
     st_ms = max_over_ranks(e0.elapsed_time(e1)) / K
     st_launches = lib.lhb200_launch_count() - l0
@@ -660,6 +674,10 @@ def run_ours(args):
             },
         }
         print(json.dumps(line))
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in outputs.items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
     if lib_comm:
         lib.lhb200_comm_destroy()
     if world > 1:
@@ -739,10 +757,16 @@ def run_reference(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed BLS steps and timed tree-hash steps (>= 1)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one returned as DIR/<name>.npy (GPU arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm; it does not apply to --impl reference")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":

@@ -1,5 +1,5 @@
 import sys, ctypes as C, os
-sys.path.insert(0, '/root/repo' if os.path.exists('/root/repo/oracle') else '.')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from oracle import bls_ref as B
 import lighthouse_b200
 from lighthouse_b200 import bls

@@ -89,6 +89,8 @@ def golden_json(name):
 
 
 def golden_validators(net):
+    """The stored SSZ validators of a genesis state: the whole list, or the list from index `stored_from` on when
+    genesis_validators.json gives one (mainnet)."""
     return lzma.open(os.path.join(GOLDEN, f"genesis_validators_{net}.bin.xz")).read()
 
 
