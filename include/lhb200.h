@@ -197,6 +197,17 @@ LHB200_API int32_t lhb200_verify_signature_sets(const uint8_t* sigs, const uint8
                                                 const uint32_t* pk_offsets, const uint64_t* rands, uint32_t n_sets,
                                                 uint8_t* ok, uint8_t* set_status);
 
+/* Many independent bls::verify_signature_sets calls in one pass.  Inputs as lhb200_verify_signature_sets, plus
+ *   group_offsets  n_groups+1 u32, CSR over the sets: group g owns sets [group_offsets[g], group_offsets[g+1])
+ * ok[g] (n_groups bytes) is exactly what lhb200_verify_signature_sets would return for group g's sets alone
+ * (empty group -> 0, blst.rs:42-44).  set_status (optional, n_sets bytes) as in lhb200_verify_signature_sets.
+ * group_offsets[0] != 0, not non-decreasing, or group_offsets[n_groups] != n_sets -> LHB200_EINVAL.
+ * Per-set verdicts are group_offsets = 0, 1, ..., n; n_groups == 1 is lhb200_verify_signature_sets itself.  Any status
+ * other than LHB200_OK leaves every ok[g] = 0.  Re-entrant like lhb200_verify_signature_sets. */
+LHB200_API int32_t lhb200_verify_signature_set_groups(const uint8_t* sigs, const uint8_t* msgs, const uint8_t* pks,
+        const uint32_t* pk_offsets, const uint64_t* rands, uint32_t n_sets,
+        const uint32_t* group_offsets, uint32_t n_groups, uint8_t* ok, uint8_t* set_status);
+
 /* Staged form of the same call (what bench.py times): create once, upload or point at device-resident inputs,
  * enqueue on a stream, read the verdict. */
 typedef struct lhb200_bls_batch lhb200_bls_batch;

@@ -207,6 +207,33 @@ inline bool verify_signature_sets(It begin, It end) {
 }
 inline bool SignatureSet::verify() const { return verify_signature_sets(this, this + 1); }
 
+/// Many independent verify_signature_sets calls in one device pass (lhb200_verify_signature_set_groups):
+/// result[g] == verify_signature_sets(groups[g]); an empty group is false.  Fails closed per group: any library error
+/// makes every element false.
+inline std::vector<bool> verify_signature_set_groups(const std::vector<std::vector<SignatureSet>>& groups) {
+    std::vector<uint8_t> sigs, msgs, pks;
+    std::vector<uint32_t> offs{0}, goffs{0};
+    for (const std::vector<SignatureSet>& group : groups) {
+        for (const SignatureSet& set : group) {
+            sigs.insert(sigs.end(), set.signature->serialize().begin(), set.signature->serialize().end());
+            msgs.insert(msgs.end(), set.message.begin(), set.message.end());
+            for (const PublicKey* pk : set.signing_keys)
+                pks.insert(pks.end(), pk->serialize_uncompressed().begin(), pk->serialize_uncompressed().end());
+            offs.push_back(static_cast<uint32_t>(pks.size() / 96));
+        }
+        goffs.push_back(static_cast<uint32_t>(offs.size() - 1));
+    }
+    const uint32_t n_groups = static_cast<uint32_t>(groups.size());
+    std::vector<uint8_t> ok(n_groups, 0);
+    const int32_t rc = lhb200_verify_signature_set_groups(sigs.data(), msgs.data(), pks.empty() ? nullptr : pks.data(),
+                                                          offs.data(), nullptr, static_cast<uint32_t>(offs.size() - 1),
+                                                          goffs.data(), n_groups, ok.data(), nullptr);
+    std::vector<bool> out(n_groups, false);
+    if (rc == LHB200_OK)
+        for (uint32_t g = 0; g < n_groups; g++) out[g] = ok[g] == 1;
+    return out;
+}
+
 /// fast_aggregate_verify / eth_fast_aggregate_verify (generic_aggregate_signature.rs:187-210)
 inline bool fast_aggregate_verify(const Signature& sig, const Hash256& msg, const std::vector<const PublicKey*>& pks) {
     if (pks.empty()) return false;

@@ -87,6 +87,7 @@ def buf(b):
 
 # ---- BLS path
 _sig("lhb200_verify_signature_sets", C.c_int32, vp, vp, vp, vp, vp, C.c_uint32, vp, vp)
+_sig("lhb200_verify_signature_set_groups", C.c_int32, vp, vp, vp, vp, vp, C.c_uint32, vp, C.c_uint32, vp, vp)
 _sig("lhb200_bls_batch_create", C.c_int32, C.c_uint32, C.c_uint64, C.POINTER(vp))
 _sig("lhb200_bls_batch_destroy", C.c_int32, vp)
 _sig("lhb200_bls_batch_upload", C.c_int32, vp, vp, vp, vp, vp, vp, C.c_uint32)

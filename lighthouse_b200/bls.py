@@ -353,6 +353,40 @@ def verify_signature_sets(sets, rands=None) -> bool:
     return verify_signature_sets_raw(sigs, msgs, pks, offs, rands)
 
 
+def verify_signature_set_groups_raw(sigs, msgs, pks, offsets, group_offsets, rands=None, want_status=False):
+    """lhb200_verify_signature_set_groups: SoA buffers as verify_signature_sets_raw plus group_offsets (uint32[G+1], CSR
+    over the sets).  -> list of G bools, each what verify_signature_sets_raw returns for that group's sets alone
+    (and the per-set statuses with want_status)."""
+    n = len(offsets) - 1
+    goffs = np.ascontiguousarray(group_offsets, dtype=np.uint32)
+    g = len(goffs) - 1
+    if g < 0:
+        raise ValueError("group_offsets needs at least one entry")
+    ok = np.zeros(max(g, 1), dtype=np.uint8)
+    st = np.zeros(max(n, 1), dtype=np.uint8)
+    offs = np.ascontiguousarray(offsets, dtype=np.uint32)
+    r = None if rands is None else np.ascontiguousarray(rands, dtype=np.uint64)
+    ps, k1 = buf(sigs if len(sigs) else b"\0")
+    pm, k2 = buf(msgs if len(msgs) else b"\0")
+    pp, k3 = buf(pks if len(pks) else b"\0")
+    check(lib.lhb200_verify_signature_set_groups(ps, pm, pp, offs.ctypes.data, None if r is None else r.ctypes.data, n,
+                                                 goffs.ctypes.data, g, ok.ctypes.data, st.ctypes.data),
+          "lhb200_verify_signature_set_groups")
+    res = [bool(v) for v in ok[:g]]
+    return (res, st[:n]) if want_status else res
+
+
+def verify_signature_set_groups(groups, rands=None) -> list:
+    """Many independent verify_signature_sets calls in one device pass: groups is a list of lists of SignatureSet;
+    element g of the result is verify_signature_sets(groups[g]) (an empty group -> False)."""
+    groups = [list(gr) for gr in groups]
+    sets = [s for gr in groups for s in gr]
+    goffs = np.zeros(len(groups) + 1, dtype=np.uint32)
+    goffs[1:] = np.cumsum([len(gr) for gr in groups], dtype=np.uint64) if groups else []
+    sigs, msgs, pks, offs = flatten_signature_sets(sets)
+    return verify_signature_set_groups_raw(sigs, msgs, pks, offs, goffs, rands)
+
+
 class ParallelSignatureSets:
     """state_processing::per_block_processing::block_signature_verifier::ParallelSignatureSets
     (block_signature_verifier.rs:84-96, :392-418): the sets of 1..N blocks are accumulated, then verified by ONE

@@ -451,6 +451,22 @@ __global__ void __launch_bounds__(BLS_BLOCK) k_fp12_reduce(const Fp12* __restric
     }
     out[t] = acc;
 }
+// out[t] = prod in[seg[t] .. seg[t+1]) (1 if empty): a product level whose chunks never cross a group boundary, so
+// that k_final_groups_warp folds a bounded number of values per group (bls/groups.cuh builds the table)
+__global__ void __launch_bounds__(BLS_BLOCK) k_fp12_reduce_seg(const Fp12* __restrict__ in, const uint32_t* __restrict__ seg,
+                                                                uint32_t n_out, Fp12* __restrict__ out) {
+    const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= n_out) return;
+    const uint32_t lo = seg[t], hi = seg[t + 1];
+    Fp12 acc;
+    if (lo < hi) acc = in[lo];
+    else fp12_set_one(acc);
+    for (uint32_t j = lo + 1; j < hi; j++) {
+        Fp12 x = in[j];
+        fp12_mul(acc, acc, x);
+    }
+    out[t] = acc;
+}
 __global__ void __launch_bounds__(BLS_BLOCK) k_g2_reduce(const G2Jac* __restrict__ in, uint32_t n, uint32_t chunk,
                                                           G2Jac* __restrict__ out) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;

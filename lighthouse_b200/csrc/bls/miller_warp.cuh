@@ -29,6 +29,18 @@ constexpr int SL = 13;                          // words per slot: odd, so lanes
 constexpr int REGION_WORDS = MW_NSLOTS * SL;    // one warp's working set (9.8 KB)
 constexpr uint32_t X_ZERO = 0, X_NEG = 2, X_DBL = 3, X_NEGDBL = 4;
 
+// Warp bodies shared with tests/hostsim (LHB_HD): a copy loop `for (w = lane; w < n; w += LANES)` is split over the 32
+// lanes on the device and run whole by the one CPU "lane" 0; warp_any is the vote over the lanes.
+#ifdef LHB_HOSTSIM
+constexpr int LANES = 1;
+#define MW_SYNCWARP() ((void)0)
+LHB_HD LHB_INLINE bool warp_any(bool v) { return v; }
+#else
+constexpr int LANES = 32;
+#define MW_SYNCWARP() __syncwarp()
+__device__ __forceinline__ bool warp_any(bool v) { return __any_sync(0xffffffffu, v); }
+#endif
+
 LHB_HD LHB_INLINE void ld(Fp& r, const uint32_t* R, int s) {
 #pragma unroll
     for (int i = 0; i < NL; i++) r.v[i] = R[s * SL + i];
@@ -175,27 +187,11 @@ LHB_HD LHB_INLINE void set_one_words(uint32_t* R, int word) {   // word < 24 * S
 
 constexpr size_t smem_bytes(int warps) { return ((size_t)warps * REGION_WORDS + table_words(MW_N_MUL, MW_N_LIN, MW_N_PHASES)) * 4; }
 #if !defined(LHB_HOSTSIM)
-// One warp per pair (P_i, H_i), i < n, plus the pair (extra_p, extra_q) = (-g1, sum r sig) as pair n.  Invalid sets
-// (status != 0, H at infinity) contribute f = 1, like k_miller_coop.  The warps of a block multiply their values
-// (dense section) and the block writes ONE Fp12.  Dynamic shared memory: smem_bytes(warps_per_block).
-__global__ void __launch_bounds__(256, 1) k_miller_warp(const G1Proj3* __restrict__ P, const G2Jac* __restrict__ H,
-                                                        const uint8_t* __restrict__ status, uint32_t n,
-                                                        const G2Jac* __restrict__ extra_q, const G1Proj3* __restrict__ extra_p,
-                                                        Fp12* __restrict__ out_f) {
-    const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-    uint32_t* R = lhb_dyn_smem + (size_t)wib * REGION_WORDS;
-    const Tables T = stage_tables(lhb_dyn_smem + (size_t)nw * REGION_WORDS, miller_tables(), MW_N_MUL, MW_N_LIN, MW_N_PHASES);
-    const uint32_t n_total = n + (extra_q ? 1u : 0u);
-    const uint32_t set = blockIdx.x * nw + wib;
+// The Miller loop of one pair by the whole warp: f (stored form, MW_S_F0_0 ...) = f_{|x|,q}(p), conjugated; f = 1 when
+// !active (warp-uniform).  Shared by k_miller_warp and k_miller_warp_pairs.
+__device__ __forceinline__ void miller_pair(uint32_t* R, int lane, const Tables& T, const G1Proj3* p, const G2Jac* q,
+                                            bool active) {
     for (int w = lane; w < 24 * SL; w += 32) set_one_words(R, w);
-    bool active = set < n_total;
-    const G2Jac* q = nullptr;
-    const G1Proj3* p = nullptr;
-    if (active) {
-        if (set >= n) { q = extra_q; p = extra_p; }
-        else { q = H + set; p = P + set; active = status[set] == 0; }
-        if (active) active = !jac_is_inf(*q);
-    }
     if (active) {   // warp-uniform
         const uint32_t* qs = reinterpret_cast<const uint32_t*>(q);     // X.c0 X.c1 Y.c0 Y.c1 Z.c0 Z.c1, 12 words each
         for (int w = lane; w < 6 * NL; w += 32) R[(MW_S_HX_0 + w / NL) * SL + w % NL] = qs[w];
@@ -215,6 +211,40 @@ __global__ void __launch_bounds__(256, 1) k_miller_warp(const G1Proj3* __restric
         }
         MW_RUN(R, lane, CONJ);
     }
+}
+
+// the warp's f (stored form) -> one Fp12 in tower order
+__device__ __forceinline__ void store_f(const uint32_t* R, int lane, Fp12* out) {
+    // w-basis coefficient k -> tower: 0 c0.c0, 1 c1.c0, 2 c0.c1, 3 c1.c1, 4 c0.c2, 5 c1.c2 (coop.cuh)
+    uint32_t* o = reinterpret_cast<uint32_t*>(out);
+    for (int w = lane; w < 12 * NL; w += 32) {
+        const int fp2_idx = w / (2 * NL), comp = (w / NL) & 1, limb = w % NL;   // tower order: c0.c0 c0.c1 c0.c2 c1.c0 c1.c1 c1.c2
+        const int k = fp2_idx < 3 ? 2 * fp2_idx : 2 * (fp2_idx - 3) + 1;
+        o[w] = R[(MW_S_F0_0 + 4 * k + comp) * SL + limb];
+    }
+}
+
+// One warp per pair (P_i, H_i), i < n, plus the pair (extra_p, extra_q) = (-g1, sum r sig) as pair n.  Invalid sets
+// (status != 0, H at infinity) contribute f = 1, like k_miller_coop.  The warps of a block multiply their values
+// (dense section) and the block writes ONE Fp12.  Dynamic shared memory: smem_bytes(warps_per_block).
+__global__ void __launch_bounds__(256, 1) k_miller_warp(const G1Proj3* __restrict__ P, const G2Jac* __restrict__ H,
+                                                        const uint8_t* __restrict__ status, uint32_t n,
+                                                        const G2Jac* __restrict__ extra_q, const G1Proj3* __restrict__ extra_p,
+                                                        Fp12* __restrict__ out_f) {
+    const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+    uint32_t* R = lhb_dyn_smem + (size_t)wib * REGION_WORDS;
+    const Tables T = stage_tables(lhb_dyn_smem + (size_t)nw * REGION_WORDS, miller_tables(), MW_N_MUL, MW_N_LIN, MW_N_PHASES);
+    const uint32_t n_total = n + (extra_q ? 1u : 0u);
+    const uint32_t set = blockIdx.x * nw + wib;
+    bool active = set < n_total;
+    const G2Jac* q = nullptr;
+    const G1Proj3* p = nullptr;
+    if (active) {
+        if (set >= n) { q = extra_q; p = extra_p; }
+        else { q = H + set; p = P + set; active = status[set] == 0; }
+        if (active) active = !jac_is_inf(*q);
+    }
+    miller_pair(R, lane, T, p, q, active);
     // product over the block's warps
     for (int stride = 1; stride < nw; stride *= 2) {
         __syncthreads();
@@ -227,14 +257,32 @@ __global__ void __launch_bounds__(256, 1) k_miller_warp(const G1Proj3* __restric
     }
     if (wib == 0) {
         __syncwarp();
-        // w-basis coefficient k -> tower: 0 c0.c0, 1 c1.c0, 2 c0.c1, 3 c1.c1, 4 c0.c2, 5 c1.c2 (coop.cuh)
-        uint32_t* o = reinterpret_cast<uint32_t*>(out_f + blockIdx.x);
-        for (int w = lane; w < 12 * NL; w += 32) {
-            const int fp2_idx = w / (2 * NL), comp = (w / NL) & 1, limb = w % NL;   // tower order: c0.c0 c0.c1 c0.c2 c1.c0 c1.c1 c1.c2
-            const int k = fp2_idx < 3 ? 2 * fp2_idx : 2 * (fp2_idx - 3) + 1;
-            o[w] = R[(MW_S_F0_0 + 4 * k + comp) * SL + limb];
-        }
+        store_f(R, lane, out_f + blockIdx.x);
     }
+}
+
+// Grouped verification: one warp per pair and ONE Fp12 per pair — no product across the warps of a block, whose pairs
+// may belong to different groups.  Pair i < n is (P_i, H_i), pair n + g is (extra_p, extra_q[g]) (-g1 and group g's
+// sum r sig).  Invalid sets and points at infinity give f = 1, as in k_miller_warp.  Any pair count: the blocks beyond
+// the resident ones run in later waves.  Dynamic shared memory: smem_bytes(warps_per_block).
+__global__ void __launch_bounds__(256, 1) k_miller_warp_pairs(const G1Proj3* __restrict__ P, const G2Jac* __restrict__ H,
+                                                              const uint8_t* __restrict__ status, uint32_t n,
+                                                              const G2Jac* __restrict__ extra_q, uint32_t n_extra,
+                                                              const G1Proj3* __restrict__ extra_p, Fp12* __restrict__ out_f) {
+    const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+    uint32_t* R = lhb_dyn_smem + (size_t)wib * REGION_WORDS;
+    const Tables T = stage_tables(lhb_dyn_smem + (size_t)nw * REGION_WORDS, miller_tables(), MW_N_MUL, MW_N_LIN, MW_N_PHASES);
+    const uint32_t k = blockIdx.x * nw + wib;
+    if (k >= n + n_extra) return;   // no block barrier below
+    const G2Jac* q;
+    const G1Proj3* p;
+    bool active = true;
+    if (k >= n) { q = extra_q + (k - n); p = extra_p; }
+    else { q = H + k; p = P + k; active = status[k] == 0; }
+    if (active) active = !jac_is_inf(*q);
+    miller_pair(R, lane, T, p, q, active);
+    __syncwarp();
+    store_f(R, lane, out_f + k);
 }
 #endif
 

@@ -14,6 +14,7 @@
 #include <sys/random.h>
 #include <vector>
 #include "bls/debug.cuh"
+#include "bls/groups.cuh"
 #include <condition_variable>
 #include <thread>
 #include "ctx.h"
@@ -92,6 +93,15 @@ struct lhb200_bls_batch {
     const uint8_t* h_pks = nullptr;          // caller's host keys (valid until result)
     int n_chunks = 0;                        // 0: inputs already complete on the device
     std::vector<uint64_t> rbuf;              // scalars drawn by the library (must outlive the async copy)
+    // grouped verification (lhb200_verify_signature_set_groups): set for the duration of one grouped call; its buffers
+    // are allocated on the first grouped call, so a handle that only runs plain verifications never holds them
+    const groups::Plan* grp = nullptr;
+    uint32_t* d_gwords = nullptr;            // the plan's tables (groups.cuh)
+    Fp12* d_pf = nullptr;                    // one Miller value per pair: n sets, then one (-g1, sum r sig) per group
+    G2Jac* d_gsum[2] = {nullptr, nullptr};   // levels of the segmented signature sums
+    Fp12* d_gfold[2] = {nullptr, nullptr};   // levels of the segmented Miller products
+    uint8_t* d_gok = nullptr;                // per-group verdicts
+    uint64_t cap_gwords = 0, cap_pf = 0, cap_gsum[2] = {}, cap_gfold[2] = {}, cap_gok = 0;
 };
 
 static void batch_free(lhb200_bls_batch* b) {
@@ -99,7 +109,8 @@ static void batch_free(lhb200_bls_batch* b) {
     if (b->d_indices) cudaFree(b->d_indices);
     void* ptrs[] = {b->d_sigs, b->d_msgs, b->d_pks, b->d_offsets, b->d_rands, b->d_sigr, b->d_sig_tmp[0],
                     b->d_sig_tmp[1], b->d_p, b->d_h, b->d_f, b->d_f_tmp[0], b->d_f_tmp[1], b->d_flast, b->d_gt,
-                    b->d_status, b->d_fail, b->d_ok, b->d_mc_scratch, b->d_neg_g1, b->d_pk_part, b->d_pk_part_bad};
+                    b->d_status, b->d_fail, b->d_ok, b->d_mc_scratch, b->d_neg_g1, b->d_pk_part, b->d_pk_part_bad,
+                    b->d_gwords, b->d_pf, b->d_gsum[0], b->d_gsum[1], b->d_gfold[0], b->d_gfold[1], b->d_gok};
     for (void* p : ptrs)
         if (p) cudaFree(p);
     if (b->h_res) cudaFreeHost(b->h_res);
@@ -275,6 +286,73 @@ void bls_shutdown() {
     g_pool_free.clear();
 }
 }  // namespace lhb200
+
+// ---- grouped verification (lhb200_verify_signature_set_groups) -------------------------------------------------------
+// The per-set stages run as in a plain call; from the sum of r sig on, every group is its own batch:
+//   s2: k_g2_sum_seg_warp levels -> one sum r sig per group
+//   s:  k_miller_warp_pairs      -> one Miller value per pair (n sets + one (-g1, sum) pair per group)
+//       k_fp12_reduce_seg levels -> at most groups::FOLD_MAX values per group (only for groups larger than that)
+//       k_final_groups_warp      -> one warp per group: fold, final exponentiation, ok[g]
+template <class T>
+static cudaError_t grow(T*& p, uint64_t& cap, uint64_t need) {
+    if (need <= cap) return cudaSuccess;
+    if (p) cudaFree(p);
+    p = nullptr;
+    cap = 0;
+    need += need / 4;
+    const cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&p), need * sizeof(T));
+    if (e == cudaSuccess) cap = need;
+    return e;
+}
+
+// Buffers of a grouped call of n sets on an idle handle.
+static int32_t group_reserve(lhb200_bls_batch* b, const groups::Plan& gp, uint32_t n) {
+    const uint32_t G = gp.n_groups;
+    LHB_CUDA(grow(b->d_gwords, b->cap_gwords, gp.words.size()));
+    LHB_CUDA(grow(b->d_pf, b->cap_pf, (uint64_t)n + G));
+    LHB_CUDA(grow(b->d_gok, b->cap_gok, G));
+    for (int k = 0; k < 2; k++) {
+        LHB_CUDA(grow(b->d_gsum[k], b->cap_gsum[k], gp.sum.max_out));
+        LHB_CUDA(grow(b->d_gfold[k], b->cap_gfold[k], gp.fold.max_out));
+    }
+    return LHB200_OK;
+}
+
+// Everything after the per-set stages of a grouped call (called by lhb200_bls_batch_verify_enqueue on stream s, once
+// the key sums, hashes and statuses are in place).
+static int32_t enqueue_group_tail(lhb200_bls_batch* b, cudaStream_t s, uint32_t n, uint64_t launches) {
+    const groups::Plan& gp = *b->grp;
+    const uint32_t G = gp.n_groups, n_pairs = n + G;
+    static const bool attr_ok = [] {
+        return cudaFuncSetAttribute(mw::k_miller_warp_pairs, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)mw::smem_bytes(mc::MC_WARPS)) == cudaSuccess &&
+               cudaFuncSetAttribute(fe::k_final_groups_warp, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)fe::groups_smem_bytes()) == cudaSuccess;
+    }();
+    if (!attr_ok) { set_error("grouped verification kernels: cannot reserve shared memory"); return LHB200_ECUDA; }
+    // four warps per block (one per scheduler) while the pairs are few, eight above (as k_miller_warp)
+    const uint32_t wpb = n_pairs <= 4 * COOP_TAIL ? 4 : mc::MC_WARPS;
+    LHB_CUDA(cudaStreamWaitEvent(s, b->e_join, 0));   // the group sums
+    LHB_CUDA(cudaEventRecord(b->e_k0, s));
+    mw::k_miller_warp_pairs<<<cdiv(n_pairs, wpb), 32 * wpb, mw::smem_bytes((int)wpb), s>>>(b->d_p, b->d_h, b->d_status, n,
+                                                                                            b->d_sig_sum, G, b->d_neg_g1, b->d_pf);
+    LHB_CUDA(cudaEventRecord(b->e_k1, s));
+    launches++;
+    const Fp12* cur = b->d_pf;
+    for (size_t l = 0; l < gp.fold.n_out.size(); l++) {
+        const uint32_t mo = gp.fold.n_out[l];
+        k_fp12_reduce_seg<<<cdiv(mo, BLS_BLOCK), BLS_BLOCK, 0, s>>>(cur, b->d_gwords + gp.fold.at[l], mo, b->d_gfold[l & 1]);
+        launches++;
+        cur = b->d_gfold[l & 1];
+    }
+    fe::k_final_groups_warp<<<cdiv(G, fe::FG_WARPS), 32 * fe::FG_WARPS, fe::groups_smem_bytes(), s>>>(
+        cur, b->d_gwords + gp.val_off_at, b->d_pf + n, b->d_status, b->d_gwords, G, b->d_gok);
+    launches++;
+    LHB_CUDA(cudaGetLastError());
+    count_launch(launches);
+    b->launches_last = launches;
+    return LHB200_OK;
+}
 
 extern "C" {
 
@@ -684,7 +762,26 @@ int32_t lhb200_bls_batch_verify_enqueue(lhb200_bls_batch* b, void* stream) {
         k_sig_prepare<<<grid, BLS_BLOCK, 0, b->s2>>>(b->in_sigs, b->in_rands, n, b->d_sigr, b->d_status, b->d_fail);
     launches++;
     LHB_CUDA(cudaEventRecord(b->e_sig, b->s2));
-    {
+    if (b->grp) {
+        // grouped: one sum r sig per group, segmented levels of four points per warp (no level when every group has one
+        // set: the set's own point is the sum)
+        const groups::Levels& L = b->grp->sum;
+        const G2Jac* cur = b->d_sigr;
+        if (!L.n_out.empty()) {
+            static const bool seg_attr_ok = [&] {
+                return cudaFuncSetAttribute(gw::k_g2_sum_seg_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)gw_smem) == cudaSuccess;
+            }();
+            if (!seg_attr_ok) { set_error("k_g2_sum_seg_warp: cannot reserve %zu B of shared memory", gw_smem); return LHB200_ECUDA; }
+        }
+        for (size_t l = 0; l < L.n_out.size(); l++) {
+            gw::k_g2_sum_seg_warp<<<cdiv(L.n_out[l], GW_WPB), 32 * GW_WPB, gw_smem, b->s2>>>(cur, b->d_gwords + L.at[l], L.n_out[l],
+                                                                                          b->d_gsum[l & 1]);
+            launches++;
+            cur = b->d_gsum[l & 1];
+        }
+        b->d_sig_sum = cur;
+        LHB_CUDA(cudaEventRecord(b->e_join, b->s2));
+    } else {
         const G2Jac* cur = b->d_sigr;
         uint32_t m = n;
         int flip = 0;
@@ -781,6 +878,7 @@ int32_t lhb200_bls_batch_verify_enqueue(lhb200_bls_batch* b, void* stream) {
         launch_pk(0, n, s);
     LHB_CUDA(cudaStreamWaitEvent(s, b->e_h2c, 0));
     LHB_CUDA(cudaStreamWaitEvent(s, b->e_sig, 0));    // the Miller kernel reads the status bytes k_sig_prepare may set
+    if (b->grp) return enqueue_group_tail(b, s, n, launches);
     static const int miller_coop = [] { const char* e = getenv("LHB_MILLER_COOP"); return e ? atoi(e) : 1; }();
     const Fp12* cur = b->d_f;
     uint32_t n_tail = 0;
@@ -1044,6 +1142,57 @@ int32_t lhb200_verify_signature_sets(const uint8_t* sigs, const uint8_t* msgs, c
     cudaStreamSynchronize(b->s2);
     cudaStreamSynchronize(b->s3);
     pool_release(b);
+    return rc;
+}
+
+// Many independent verify_signature_sets calls in one pass: group g owns sets [group_offsets[g], group_offsets[g+1])
+// and ok[g] is what lhb200_verify_signature_sets would return for those sets alone (an empty group: 0).  What
+// Lighthouse's batch fallbacks need (attestation_verification/batch.rs): one call that names the bad items instead of one
+// call per item.  The per-set stages are shared; sums, Miller products and final exponentiations are per group.
+int32_t lhb200_verify_signature_set_groups(const uint8_t* sigs, const uint8_t* msgs, const uint8_t* pks,
+                                           const uint32_t* pk_offsets, const uint64_t* rands, uint32_t n_sets,
+                                           const uint32_t* group_offsets, uint32_t n_groups, uint8_t* ok,
+                                           uint8_t* set_status) {
+    LHB_REQUIRE_READY();
+    if (!group_offsets || (n_groups && !ok)) { set_error("verify_signature_set_groups: null argument"); return LHB200_EINVAL; }
+    if (n_groups) memset(ok, 0, n_groups);
+    if (group_offsets[0] != 0 || group_offsets[n_groups] != n_sets) {
+        set_error("verify_signature_set_groups: group offsets must run from 0 to n_sets");
+        return LHB200_EINVAL;
+    }
+    for (uint32_t g = 0; g < n_groups; g++)
+        if (group_offsets[g] > group_offsets[g + 1]) { set_error("verify_signature_set_groups: group offsets not monotone"); return LHB200_EINVAL; }
+    if (n_sets == 0) return LHB200_OK;   // every group is empty
+    // one group: the plain single-verdict path
+    if (n_groups == 1) return lhb200_verify_signature_sets(sigs, msgs, pks, pk_offsets, rands, n_sets, ok, set_status);
+    if (!pk_offsets) { set_error("verify_signature_set_groups: null offsets"); return LHB200_EINVAL; }
+    groups::Plan plan;
+    groups::build_plan(plan, group_offsets, n_groups);
+    lhb200_bls_batch* b = pool_acquire(n_sets, pk_offsets[n_sets]);
+    if (!b) return LHB200_ENOMEM;
+    int32_t rc = group_reserve(b, plan, n_sets);
+    if (!rc) rc = lhb200_bls_batch_upload_async(b, sigs, msgs, pks, pk_offsets, rands, n_sets, b->s_main);
+    if (!rc) {
+        const cudaError_t e = cudaMemcpyAsync(b->d_gwords, plan.words.data(), plan.words.size() * 4, cudaMemcpyHostToDevice, b->s_main);
+        if (e != cudaSuccess) rc = cuda_fail(e, "group plan upload");
+    }
+    if (!rc) {
+        b->grp = &plan;
+        rc = lhb200_bls_batch_verify_enqueue(b, b->s_main);
+        b->grp = nullptr;
+    }
+    if (!rc) {   // (there may be more groups than the handle's pinned result buffer holds: straight to the caller)
+        cudaError_t e = cudaMemcpyAsync(ok, b->d_gok, n_groups, cudaMemcpyDeviceToHost, b->s_main);
+        if (e == cudaSuccess && set_status)
+            e = cudaMemcpyAsync(set_status, b->d_status, n_sets, cudaMemcpyDeviceToHost, b->s_main);
+        if (e == cudaSuccess) e = cudaStreamSynchronize(b->s_main);
+        if (e != cudaSuccess) rc = cuda_fail(e, "grouped verdicts");
+    }
+    cudaStreamSynchronize(b->s_main);   // `plan` must outlive its upload
+    cudaStreamSynchronize(b->s2);
+    cudaStreamSynchronize(b->s3);
+    pool_release(b);
+    if (rc && n_groups) memset(ok, 0, n_groups);
     return rc;
 }
 

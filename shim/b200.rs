@@ -51,6 +51,18 @@ extern "C" {
         ok: *mut u8,
         set_status: *mut u8,
     ) -> i32;
+    fn lhb200_verify_signature_set_groups(
+        sigs: *const u8,
+        msgs: *const u8,
+        pks: *const u8,
+        pk_offsets: *const u32,
+        rands: *const u64,
+        n_sets: u32,
+        group_offsets: *const u32,
+        n_groups: u32,
+        ok: *mut u8,
+        set_status: *mut u8,
+    ) -> i32;
     fn lhb200_aggregate_verify(sig96: *const u8, msgs: *const u8, pks96: *const u8, n: u32, ok: *mut u8) -> i32;
     fn lhb200_g2_aggregate(sigs96: *const u8, n: u32, out96: *mut u8) -> i32;
     fn lhb200_g1_aggregate(pks96: *const u8, n: u32, out48: *mut u8, out96: *mut u8) -> i32;
@@ -80,6 +92,7 @@ const CURVE_ORDER_BE: [u8; 32] = [
 
 /// Provides the externally-facing, core BLS types.
 pub mod types {
+    pub use super::verify_signature_set_groups;
     pub use super::verify_signature_sets;
     pub use super::AggregatePublicKey;
     pub use super::AggregateSignature;
@@ -143,6 +156,56 @@ pub fn verify_signature_sets<'a>(signature_sets: impl ExactSizeIterator<Item = &
         )
     };
     rc == 0 && ok == 1
+}
+
+/// Many independent `verify_signature_sets` calls in one device pass (`lhb200_verify_signature_set_groups`): element g
+/// is `verify_signature_sets(groups[g].iter())`, an empty group is false.  What the batch fallbacks of
+/// `attestation_verification/batch.rs` need: one call that names the bad items.  Fails closed: any library error makes
+/// every element false.  An "empty" signature or a set without keys fails its own group only (the device reports them).
+pub fn verify_signature_set_groups(groups: &[&[SignatureSet]]) -> Vec<bool> {
+    let n_groups = groups.len();
+    let n: usize = groups.iter().map(|g| g.len()).sum();
+    let mut sigs = Vec::with_capacity(n * SIGNATURE_BYTES_LEN);
+    let mut msgs = Vec::with_capacity(n * 32);
+    let mut offsets: Vec<u32> = Vec::with_capacity(n + 1);
+    let mut group_offsets: Vec<u32> = Vec::with_capacity(n_groups + 1);
+    let n_keys: usize = groups.iter().flat_map(|g| g.iter()).map(|s| s.signing_keys.len()).sum();
+    let mut pks = Vec::with_capacity(n_keys * PUBLIC_KEY_UNCOMPRESSED_BYTES_LEN);
+    offsets.push(0);
+    group_offsets.push(0);
+    for group in groups {
+        for set in group.iter() {
+            match set.signature.point() {
+                Some(point) => sigs.extend_from_slice(&point.0),
+                None => sigs.extend_from_slice(&[0u8; SIGNATURE_BYTES_LEN]), // "empty": status 1 on the device
+            }
+            msgs.extend_from_slice(set.message.as_bytes());
+            for pk in set.signing_keys.iter() {
+                pks.extend_from_slice(&pk.point().uncompressed);
+            }
+            offsets.push((pks.len() / PUBLIC_KEY_UNCOMPRESSED_BYTES_LEN) as u32);
+        }
+        group_offsets.push((offsets.len() - 1) as u32);
+    }
+    let mut ok = vec![0u8; n_groups];
+    if n == 0 || !ensure_init() {
+        return vec![false; n_groups];
+    }
+    let rc = unsafe {
+        lhb200_verify_signature_set_groups(
+            sigs.as_ptr(),
+            msgs.as_ptr(),
+            pks.as_ptr(),
+            offsets.as_ptr(),
+            std::ptr::null(),
+            n as u32,
+            group_offsets.as_ptr(),
+            n_groups as u32,
+            ok.as_mut_ptr(),
+            std::ptr::null_mut(),
+        )
+    };
+    ok.iter().map(|&v| rc == 0 && v == 1).collect()
 }
 
 /// One set, explicit keys: `Signature::verify` / `fast_aggregate_verify` (blst.rs:196-200, :250-261).
